@@ -401,6 +401,39 @@ def parity_block(pkg, ctx, n):
     return out
 
 
+DUMP_CHUNKS, DUMP_CHUNK_WORDS = 256, 4096          # 1 Mi words of the probe buffer: 8 MiB as float64
+
+
+def dump_chunks():
+    """First word of each chunk of the probe buffer that --dump-outputs samples: fixed, seeded, ascending."""
+    import numpy as np
+    rng = np.random.default_rng(0)
+    return [int(c) * DUMP_CHUNK_WORDS for c in np.sort(rng.choice(S_BYTES // 4 // DUMP_CHUNK_WORDS, DUMP_CHUNKS, replace=False))]
+
+
+def probe_outputs(ctx, res):
+    """What the value leg's last step returned (--dump-outputs), as float64 arrays.  64-bit integers are split into
+    [high, low] 32-bit halves so that float64 holds them exactly; timings are left out, they differ from run to run.
+    probe_buffer_sample: the dump_chunks() of the 1 GiB buffer the step wrote (what the next pass verifies)."""
+    import numpy as np
+
+    def u64(values):
+        return [[v >> 32, v & 0xFFFFFFFF] for v in values]
+    return {"probe_seed": [r.seed for r in res], "probe_checksum": u64(r.checksum for r in res),
+            "probe_expected_checksum": u64(r.expected_checksum for r in res),
+            "probe_mismatches": u64(r.mismatches for r in res), "probe_first_bad_word": u64(r.first_bad_word for r in res),
+            "probe_bytes": u64(r.bytes for r in res), "probe_healthy": [float(r.healthy) for r in res],
+            "probe_err": [r.err for r in res],
+            "probe_buffer_sample": np.concatenate([ctx.probe_peek(0, w, DUMP_CHUNK_WORDS) for w in dump_chunks()])}
+
+
+def write_outputs(directory, outputs):
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(directory, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 class FileFlag:
     """Rank 0 works alone while the other ranks sleep on a file (an NCCL barrier would park a spinning kernel on
     every GPU that rank 0 is about to measure)."""
@@ -433,7 +466,9 @@ def main():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200")
     ap.add_argument("--variant", type=int, default=0, help="0 = TMA-staged kernel (default), 1 = register path")
-    ap.add_argument("--single-cycles", type=int, default=0, help="cycles of the single-process leg (default max(steps, 500))")
+    ap.add_argument("--single-cycles", type=int, default=0, help="cycles of the single-process leg (default --steps)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step returned as DIR/<name>.npy (float64)")
     args = ap.parse_args()
     # stdout carries exactly ONE JSON line: libraries (NCCL prints its version banner there) are
     # diverted to stderr for the whole run and the line is written to the saved descriptor.
@@ -445,6 +480,8 @@ def main():
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs dumps the B200 arm's outputs; the reference arm has none to compare")
         run_reference(args, rank, world)
         return
     warmup = max(3, args.warmup)
@@ -477,7 +514,13 @@ def main():
 
     barrier()   # pays the NCCL communicator init before any warm-up
     # ---- value leg: the probe through the C ABI, buffers resident ------------------------------
-    warm(lambda: ctx.probe_health(variant=args.variant))
+    # Every pass re-keys the buffer with the next seed, so the timed passes' inputs depend on how many passes came
+    # before them.  The time-bounded warm-up therefore runs on a scratch context over the same GPU, and the measured
+    # context runs exactly `warmup` passes: its inputs, and so its results, follow from the arguments alone.
+    with pkg.Context(ctx.uri) as scratch:
+        warm(lambda: scratch.probe_health(variant=args.variant))
+    for _ in range(warmup):
+        ctx.probe_health(variant=args.variant)
     barrier()
     kernel_ms, unhealthy, value_ms, fracs = [], 0, [], []
     w0 = time.monotonic_ns()
@@ -493,6 +536,7 @@ def main():
     t_value = time.perf_counter() - t0
     windows.append((w0, time.monotonic_ns()))
     gbs_ref = res[0].gbs_ref
+    outputs = probe_outputs(ctx, res) if args.dump_outputs and rank == 0 else None
     barrier()
     t_value = max_over_ranks(t_value)
 
@@ -547,6 +591,8 @@ def main():
     e2e_p99_max_rank = max_over_ranks(pctl(e2e_ms, 0.99))
     msg = pkg.v1beta1.ListAndWatchResponse.FromString(wire)
     assert len(msg.devices) == 1 and msg.devices[0].health == "Healthy", msg
+    if outputs is not None:
+        outputs["list_and_watch_healthy"] = [float(d.health == "Healthy") for d in msg.devices]
 
     # ---- stream start: the initial ListAndWatch list (enumerate + homogeneity + encode; the reference does
     # two GetAMDGPUs() walks here, plugin.go:231,237) -- reported next to reference_cpu_path ------
@@ -597,7 +643,7 @@ def main():
     if rank == 0:
         try:
             w0 = time.monotonic_ns()
-            cycles = args.single_cycles or max(args.steps, 500)
+            cycles = args.single_cycles or args.steps
             sctx, sp, p2p = single_process_leg(pkg, world, cycles, warmup, args.variant)
             windows.append((w0, time.monotonic_ns()))
             try:
@@ -685,6 +731,8 @@ def main():
     line["cpu_baseline"] = {"value": round(cpu_gbs, 2), "unit": UNIT, "cores": threads, "kind": "port",
                             "sample": "the 1 GiB probe buffer of ONE device, %d passes in %.1f s, host DRAM, %d threads" % (passes, dt, threads),
                             "cycle_ms_kfd_walk": round(start_ms, 4), "kfd_walk_heartbeat_ms": round(beat_ms, 4)}
+    if outputs is not None:
+        write_outputs(args.dump_outputs, outputs)
     print(json.dumps(line), flush=True)
     rg.close()
     bad = [k for k, v in (parity or {}).items() if v is False]

@@ -5,6 +5,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -39,6 +41,43 @@ def test_product_arm_refuses_to_run_without_a_gpu():
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "1"], capture_output=True, text=True,
                        timeout=300, cwd=ROOT)
     assert r.returncode != 0 and "no CPU fallback" in (r.stderr + r.stdout)
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_last_timed_pass(tmp_path):
+    """--dump-outputs writes what the value leg's last timed pass returned.  The measured context runs exactly --warmup
+    passes and then --steps timed ones, so that pass verified the seed W+K-1 steps after the initial one whatever the
+    warm-up's time floor did, and its results and the buffer it re-keyed equal the oracle's."""
+    import numpy as np
+    from oracle import probe as oprobe
+    sys.path.insert(0, ROOT)
+    import bench
+    out = tmp_path / "dump"
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--steps", "4", "--warmup", "3",
+                        "--dump-outputs", str(out)], capture_output=True, text=True, timeout=900, cwd=ROOT)
+    assert r.returncode == 0, r.stderr[-3000:]
+    d = json.loads(r.stdout.strip().splitlines()[-1])
+    assert d["steps"] == 4 and d["warmup"] == 3 and d["single_process"]["cycles"] == 4
+    assert sum(f.stat().st_size for f in out.iterdir()) <= 64 << 20
+
+    def load(name):
+        a = np.load(out / (name + ".npy"))
+        assert a.dtype == np.float64
+        return a
+
+    def u64(name):
+        return [int(hi) << 32 | int(lo) for hi, lo in load(name)]
+    seed = oprobe.initial_seed(0)
+    for _ in range(3 + 4 - 1):
+        seed = oprobe.next_seed(seed)
+    n_words = bench.S_BYTES // 4
+    assert load("probe_seed").tolist() == [seed]
+    assert u64("probe_checksum") == u64("probe_expected_checksum") == [oprobe.expected_checksum(n_words, seed)]
+    assert (u64("probe_mismatches"), u64("probe_first_bad_word"), u64("probe_bytes")) == ([0], [oprobe.NO_BAD], [2 * bench.S_BYTES])
+    assert load("probe_healthy").tolist() == [1.0] and load("probe_err").tolist() == [0.0]
+    assert load("list_and_watch_healthy").tolist() == [1.0]
+    want = np.concatenate([oprobe.pattern(bench.DUMP_CHUNK_WORDS, oprobe.next_seed(seed), w) for w in bench.dump_chunks()])
+    assert np.array_equal(load("probe_buffer_sample"), want.astype(np.float64))
 
 
 def test_product_never_imports_links_or_executes_the_oracle():
