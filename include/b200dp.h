@@ -184,6 +184,12 @@ typedef struct b2dp_ctx b2dp_ctx;
  *                     pass is armed, its stream wait stalls all other GPU work THIS PROCESS submits to that GPU (other streams,
  *                     a second context of this library; measured) -- other processes are not affected (a tenant's kernels
  *                     keep their latency).  Use it only where the library is the process's sole user of the GPU (the daemon).
+ *                     compute=0|1 (default 0): after every probe pass, each GPU whose HBM pass ran also runs the tensor-core
+ *                     check (b2dp_compute_check with default options: tcgen05 bf16 and e4m3 GEMM tiles on every SM, verified
+ *                     bit for bit against host hashes); wrong data, a launch failure or a missed deadline makes that pass
+ *                     Unhealthy with B2DP_RES_COMPUTE, reported once (the next pass runs fresh).  busy=skip skips it with the
+ *                     pass; it travels through probe=helpers.  compute=1 turns prearm=1 off: a check queued behind an armed
+ *                     stream wait would stall until the next heartbeat.
  *                     seed_index=<i>: (helpers) the enumeration index this one-device context stands for.
  *                     A GPU whose own setup fails (or that break=<i>+<j>, a test hook, names by enumeration index)
  *                     stays in the device list and is reported Unhealthy with B2DP_E_CUDA on every pass; the open
@@ -266,6 +272,8 @@ typedef struct b2dp_probe_result {
 #define B2DP_RES_SLOW 0x80u        /* achieved GB/s was below min_gbs_applied */
 #define B2DP_RES_PREARMED 0x100u   /* prearm=1: this pass had been enqueued behind its doorbell while the previous one ran; the
                                       heartbeat only rang the doorbell (no launch on its critical path) */
+#define B2DP_RES_COMPUTE 0x200u   /* compute=1: the tensor-core check after the pass failed (wrong product, launch failure or missed
+                                      deadline) => Unhealthy; not debounced, not sticky */
 #define B2DP_RES_XID 0x8u          /* xid=1: a critical Xid event was delivered for this device since open (or the
                                       last b2dp_probe_reset) => Unhealthy, sticky */
 
@@ -304,6 +312,60 @@ B2DP_API int b2dp_expected_checksum(uint64_t n_words, uint32_t seed, uint64_t *c
 /* Copy `n_words` words starting at `word_index` of the buffer the next probe will read
  * (parity tests compare it with the oracle's pattern). */
 B2DP_API int b2dp_probe_peek(b2dp_ctx *ctx, int device, uint64_t word_index, uint32_t *out, uint64_t n_words);
+
+/* ---- tensor-core check (extends the per-GPU verdict of exporter/health.go:42-82) ----------------------------------
+ * One CTA per SM runs T tiles of M=128 N=128 K=128 on the tensor cores (tcgen05.mma, fp32 accumulators in tensor
+ * memory) for each of two kinds, back to back: kind::f16 with bf16 operands (kind 0) and kind::f8f6f4 with e4m3
+ * operands (kind 1).  Operands are integers in [-7, 7] from a per-device seed, so every product is exact; each
+ * accumulator row is hashed on the device and compared with the hash the host computed at open. */
+typedef struct b2dp_compute_opts {
+    uint32_t timeout_ms;   /* 0 = 5000 */
+    uint32_t tiles;        /* tiles per CTA per kind; 0 = the default (B2DP_COMPUTE_DEFAULT_TILES) */
+    uint32_t flags;        /* B2DP_COMPUTE_EVENT_TIMING */
+    uint32_t reserved;
+} b2dp_compute_opts;
+#define B2DP_COMPUTE_EVENT_TIMING 0x20u   /* also bracket the two launches with CUDA events and report ms_event */
+#define B2DP_COMPUTE_DEFAULT_TILES 8u
+#define B2DP_COMPUTE_MAX_TILES 65536u
+
+typedef struct b2dp_compute_result {
+    int32_t device;             /* index into b2dp_enumerate() order */
+    int32_t healthy;            /* 1: every row of every tile matched */
+    int32_t err;                /* B2DP_OK | B2DP_E_CUDA (launch failed / no sequence echo) | B2DP_E_TIMEOUT */
+    uint32_t seed;              /* operand pool seed of this device */
+    int32_t sms;                /* SMs of the device */
+    int32_t sms_covered;        /* SMs that ran a CTA of both kinds (a tenant may hold some: reported, not a verdict) */
+    int32_t sms_failed;         /* SMs with at least one bad row */
+    int32_t first_bad_sm;       /* lowest %smid with a bad row, -1 if none */
+    int32_t first_bad_kind;     /* on first_bad_sm: 0 bf16, 1 e4m3; -1 if none */
+    int32_t first_bad_tile;     /* on first_bad_sm, in that kind: the first tile with a bad row; -1 if none */
+    int32_t first_bad_row;      /* its first bad row; -1 if none */
+    uint32_t reserved0;
+    uint64_t tiles;             /* tiles verified over both kinds and all SMs */
+    uint64_t bad_rows;          /* accumulator rows whose hash did not match */
+    uint32_t bad_sm_mask[8];    /* bit s (word s / 32) = %smid s had a bad row */
+    uint32_t covered_mask[8];   /* bit s = %smid s ran a CTA of both kinds */
+    float ms_device;            /* %globaltimer span: first CTA start .. result published */
+    float ms_event;             /* CUDA-event time of both launches (B2DP_COMPUTE_EVENT_TIMING), else 0 */
+    float tflops;               /* 2*128*128*128 * tiles over ms_event if timed, else over ms_device (reported, not judged) */
+    uint32_t reserved1;
+} b2dp_compute_result;
+
+/* exporter/health.go:42-82 (the per-GPU verdict) and the heartbeat that carries it, plugin.go:304-320: run the
+ * tensor-core check on every GPU of the context concurrently and return per-SM detail.  Works whether or not the
+ * context was opened with compute=1.  A device that could not be set up gets err = B2DP_E_CUDA and is not launched on.
+ * B2DP_E_UNSUPPORTED on kfd:, synthetic:, probe=off and probe=helpers (MIG) contexts. */
+B2DP_API int b2dp_compute_check(b2dp_ctx *ctx, const b2dp_compute_opts *opts, b2dp_compute_result *out, int cap, int *n);
+/* Bit-exact parity hook for the verdict of exporter/health.go:42-82: one CTA computes one tile C = A[a_set] . B[b_set]^T
+ * of `kind` (0 bf16, 1 e4m3) from the device's pool and returns the raw fp32 accumulator, row-major [128][128]. */
+B2DP_API int b2dp_compute_tile(b2dp_ctx *ctx, int device, int kind, int a_set, int b_set, float *c);
+/* Test hook for the verdict of exporter/health.go:42-82, as b2dp_probe_inject_fault: in the next check on `device`
+ * (b2dp_compute_check or a compute=1 pass) the CTA on %smid `sm` XORs `mask` into row 0, column 0 of its first bf16
+ * tile after reading it from tensor memory -- a simulated wrong product, no GPU fault.  One-shot. */
+B2DP_API int b2dp_compute_inject_fault(b2dp_ctx *ctx, int device, int sm, uint32_t mask);
+/* The host reference behind the verdict of exporter/health.go:42-82: the 128 row hashes of tile (a_set, b_set) of
+ * `kind` for pool `seed` (oracle/tc_check.py).  No context, no GPU.  cap >= 128. */
+B2DP_API int b2dp_compute_expected(uint32_t seed, int kind, int a_set, int b_set, uint64_t *row_hash, int cap, int *n);
 
 /* exporter/health.go:86-106 PopulatePerGPUDHealth(devs, defaultHealth) merge rule.
  * have_source = 0 reproduces "exporter socket absent / RPC failed" (every device gets the

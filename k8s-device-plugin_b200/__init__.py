@@ -11,6 +11,6 @@ All arithmetic happens in libb200dp.so (C++/CUDA); nothing here imports `oracle/
 """
 from . import _native  # noqa: F401  (raises if libb200dp.so is missing: no fallback)
 from . import allocator, amdgpu, exporter, labeller, plugin, synth, v1beta1  # noqa: F401
-from .context import Context  # noqa: F401
+from .context import Context, compute_expected  # noqa: F401
 
 __all__ = ["Context", "amdgpu", "allocator", "plugin", "exporter", "labeller"]

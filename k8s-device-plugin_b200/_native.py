@@ -37,6 +37,10 @@ PROBE_VIA_WORKERS = 0x10
 PROBE_EVENT_TIMING = 0x20
 RES_SKIPPED_BUSY, RES_SHRUNK, RES_ECC, RES_XID, RES_SMALL_RING = 1, 2, 4, 8, 16
 RES_CONTENDED, RES_NO_FLOOR, RES_SLOW, RES_PREARMED = 0x20, 0x40, 0x80, 0x100
+RES_COMPUTE = 0x200
+COMPUTE_EVENT_TIMING = 0x20
+COMPUTE_DEFAULT_TILES, COMPUTE_MAX_TILES = 8, 65536
+COMPUTE_KIND_BF16, COMPUTE_KIND_E4M3 = 0, 1
 LW_INITIAL, LW_HEARTBEAT, LW_EXTERNAL_SOURCE, LW_NO_PROBE, LW_LINK_CHECK = 1, 2, 4, 8, 16
 
 Id64 = C.c_char * 64
@@ -103,6 +107,19 @@ class ProbeInfo(C.Structure):
                 ("uuid", C.c_char * 48), ("name", C.c_char * 64)]
 
 
+class ComputeOpts(C.Structure):
+    _fields_ = [("timeout_ms", C.c_uint32), ("tiles", C.c_uint32), ("flags", C.c_uint32), ("reserved", C.c_uint32)]
+
+
+class ComputeResult(C.Structure):
+    _fields_ = [("device", C.c_int32), ("healthy", C.c_int32), ("err", C.c_int32), ("seed", C.c_uint32),
+                ("sms", C.c_int32), ("sms_covered", C.c_int32), ("sms_failed", C.c_int32), ("first_bad_sm", C.c_int32),
+                ("first_bad_kind", C.c_int32), ("first_bad_tile", C.c_int32), ("first_bad_row", C.c_int32),
+                ("reserved0", C.c_uint32), ("tiles", C.c_uint64), ("bad_rows", C.c_uint64),
+                ("bad_sm_mask", C.c_uint32 * 8), ("covered_mask", C.c_uint32 * 8), ("ms_device", C.c_float),
+                ("ms_event", C.c_float), ("tflops", C.c_float), ("reserved1", C.c_uint32)]
+
+
 class P2pOpts(C.Structure):
     _fields_ = [("bytes", C.c_uint64), ("iters", C.c_uint32), ("flags", C.c_uint32)]
 
@@ -148,6 +165,10 @@ SIGNATURES = {
     "b2dp_probe_set_ref": (_i, [_vp, _i, C.c_float]),
     "b2dp_probe_describe": (_i, [_vp, _i, _P(ProbeInfo)]),
     "b2dp_expected_checksum": (_i, [C.c_uint64, C.c_uint32, _P(C.c_uint64)]),
+    "b2dp_compute_check": (_i, [_vp, _P(ComputeOpts), _P(ComputeResult), _i, _ip]),
+    "b2dp_compute_tile": (_i, [_vp, _i, _i, _i, _i, _P(C.c_float)]),
+    "b2dp_compute_inject_fault": (_i, [_vp, _i, _i, C.c_uint32]),
+    "b2dp_compute_expected": (_i, [C.c_uint32, _i, _i, _i, _P(C.c_uint64), _i, _ip]),
     "b2dp_merge_health": (_i, [_P(Id64), _i, C.c_int32, _i, _P(Id64), _i32p, _i, _i32p]),
     "b2dp_list_and_watch": (_i, [_vp, _cp, _P(CycleOpts), _u8p, C.c_size_t, _szp, _P(CycleStats)]),
     "b2dp_watch_start": (_i, [_vp, _cp, C.c_uint32, _P(CycleOpts), WatchCb, _vp, _P(_vp)]),

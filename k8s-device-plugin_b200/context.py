@@ -46,6 +46,43 @@ class CycleStats:
     probe_frac_min: float = 0.0
 
 
+@dataclass
+class ComputeResult:
+    """One device's tensor-core check (b2dp_compute_result); masks are ints with bit s = %smid s."""
+    device: int
+    healthy: bool
+    err: int
+    seed: int
+    sms: int
+    sms_covered: int
+    sms_failed: int
+    first_bad_sm: int
+    first_bad_kind: int
+    first_bad_tile: int
+    first_bad_row: int
+    tiles: int
+    bad_rows: int
+    bad_sm_mask: int
+    covered_mask: int
+    ms_device: float
+    ms_event: float
+    tflops: float
+
+
+def _mask(words) -> int:
+    return sum(int(w) << (32 * i) for i, w in enumerate(words))
+
+
+def compute_expected(seed: int, kind: int, a_set: int, b_set: int):
+    """The host's 128 row hashes of tile (a_set, b_set) (b2dp_compute_expected; no context, no GPU)."""
+    import numpy as np
+    out = np.zeros(128, dtype=np.uint64)
+    n = C.c_int()
+    N.check(N.lib.b2dp_compute_expected(seed, kind, a_set, b_set, out.ctypes.data_as(C.POINTER(C.c_uint64)), 128,
+                                        C.byref(n)))
+    return out[:n.value]
+
+
 class Context:
     def __init__(self, uri: str):
         self.uri = uri
@@ -155,6 +192,30 @@ class Context:
         N.check(N.lib.b2dp_probe_peek(self._h, device, word_index, out.ctypes.data_as(C.POINTER(C.c_uint32)), n_words),
                 self._h)
         return out
+
+    # ---- tensor-core check ---------------------------------------------------------------
+    def compute_check(self, tiles: int = 0, timeout_ms: int = 0, timed: bool = False) -> List[ComputeResult]:
+        """The tensor-core check on every GPU at once (b2dp_compute_check), with per-SM detail."""
+        opts = N.ComputeOpts(timeout_ms, tiles, N.COMPUTE_EVENT_TIMING if timed else 0, 0)
+        rc, arr, n = N.grow_call(lambda cap: (N.ComputeResult * cap)(),
+                                 lambda a, cap, pn: N.lib.b2dp_compute_check(self._h, C.byref(opts), a, cap, pn))
+        N.check(rc, self._h)
+        return [ComputeResult(r.device, bool(r.healthy), r.err, r.seed, r.sms, r.sms_covered, r.sms_failed,
+                              r.first_bad_sm, r.first_bad_kind, r.first_bad_tile, r.first_bad_row, r.tiles, r.bad_rows,
+                              _mask(r.bad_sm_mask), _mask(r.covered_mask), r.ms_device, r.ms_event, r.tflops)
+                for r in arr[:n]]
+
+    def compute_tile(self, device: int, kind: int, a_set: int, b_set: int):
+        """One tile C = A[a_set] . B[b_set]^T of `kind` on one CTA: the raw fp32 accumulator, [128, 128]."""
+        import numpy as np
+        c = np.zeros((128, 128), dtype=np.float32)
+        N.check(N.lib.b2dp_compute_tile(self._h, device, kind, a_set, b_set, c.ctypes.data_as(C.POINTER(C.c_float))),
+                self._h)
+        return c
+
+    def compute_inject_fault(self, device: int, sm: int, mask: int):
+        """One-shot: the next check on `device` flips `mask` into one accumulator word on %smid `sm`."""
+        N.check(N.lib.b2dp_compute_inject_fault(self._h, device, sm, mask), self._h)
 
     # ---- ListAndWatch --------------------------------------------------------------------
     def list_and_watch(self, resource: str = "gpu", flags: int = N.LW_INITIAL, external: Optional[Dict[str, bool]] = None,

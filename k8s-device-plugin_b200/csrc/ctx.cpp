@@ -52,6 +52,11 @@ struct b2dp_ctx {
 
 static int fail(int code, const std::string& msg) { t_last_error = msg; return code; }
 
+namespace b2dp {
+CudaBackend* ctx_cuda_backend(b2dp_ctx* c) { return c && c->kind == b2dp_ctx::CUDA ? c->cuda : nullptr; }
+int ctx_fail(int code, const std::string& msg) { return fail(code, msg); }
+}  // namespace b2dp
+
 static int enumerate_ctx(b2dp_ctx* c, std::vector<Device>& devs) {
     std::string err;
     int rc = c->kind == b2dp_ctx::KFD ? kfd_enumerate(c->sysroot, devs, err) : cuda_enumerate(c->cuda, devs, err);
@@ -245,6 +250,11 @@ extern "C" int b2dp_open(const char* uri, b2dp_ctx** out) {
             } else if (p.first == "shrink_bytes") cfg.shrink_bytes = strtoull(p.second.c_str(), nullptr, 0);
             else if (p.first == "ecc") cfg.check_ecc = p.second != "0";
             else if (p.first == "xid") cfg.check_xid = p.second != "0";
+            else if (p.first == "compute") {
+                if (p.second == "0") cfg.compute = false;
+                else if (p.second == "1") cfg.compute = true;
+                else return fail(B2DP_E_INVAL, "compute= wants 0|1");
+            }
             else if (p.first == "break") {
                 size_t pos = 0;
                 while (pos <= p.second.size()) {
@@ -260,7 +270,7 @@ extern "C" int b2dp_open(const char* uri, b2dp_ctx** out) {
         if (cfg.bytes < 4096 || cfg.bytes % 16) return fail(B2DP_E_INVAL, "bytes must be a multiple of 16, >= 4096");
         if (cfg.mig_bytes < 4096 || cfg.mig_bytes % 16) return fail(B2DP_E_INVAL, "mig_bytes must be a multiple of 16, >= 4096");
         // what every helper process inherits: the verdict-related options (the ring geometry is set per unit)
-        for (const char* k : {"min_gbs", "min_frac", "ref_gbs", "calib", "slow_passes", "prearm", "busy", "shrink_bytes", "ecc"}) {
+        for (const char* k : {"min_gbs", "min_frac", "ref_gbs", "calib", "slow_passes", "prearm", "busy", "shrink_bytes", "ecc", "compute"}) {
             auto it = kv.find(k);
             if (it != kv.end()) cfg.passthrough += std::string(",") + k + "=" + it->second;
         }

@@ -33,6 +33,7 @@
 #include "internal.hpp"
 #include "nvml_dyn.hpp"
 #include "pattern_math.hpp"
+#include "tc_check.cuh"
 #include "units_backend.hpp"
 
 namespace b2dp {
@@ -127,6 +128,19 @@ struct Gpu {
     unsigned long long seq = 0;
     std::atomic<bool> inflight{false};  // a timed-out pass is still owned by the worker
     std::vector<char> peer_enabled;
+    int seed_idx = 0;                   // the index the per-device seeds derive from
+    // tensor-core check (tc_check.cuh); set up at open with compute=1, else on first use
+    bool tc_ready = false;
+    uint32_t tc_seed = 0;
+    uint8_t* tc_pool[2] = {nullptr, nullptr};  // per kind: operand tiles (UMMA layout) + row-hash table
+    TcCtl* tc_ctl = nullptr;
+    TcOut *tc_out_h = nullptr, *tc_out_d = nullptr;
+    float* tc_c = nullptr;              // b2dp_compute_tile's accumulator
+    cudaEvent_t tc_e0 = nullptr, tc_e1 = nullptr;
+    unsigned long long tc_seq = 0;
+    uint32_t tc_check_no = 0;           // advances the combination schedule
+    int tc_fault_sm = -1;               // b2dp_compute_inject_fault: one-shot
+    uint32_t tc_fault_mask = 0;
 };
 
 // launchers=2: a second launcher thread enqueues the passes of the GPUs on the OTHER NUMA node while the caller
@@ -334,6 +348,192 @@ static void probe_collect(Gpu* g, ProbeJobResult* r) {
         hbm_fill<256><<<(int)g->sms * 8, 256, 0, g->stream>>>(g->buf[g->cur], n_vec, g->seed);
         cudaStreamSynchronize(g->stream);
     }
+}
+
+// ---- tensor-core check (tc_check.cuh) ---------------------------------------------------------------------------------
+// Runs on g's worker: the operand pools and the expected row hashes are computed on the HOST (tc_math.hpp) and copied
+// once; the device under test never computes its own reference.
+static cudaError_t tc_setup(Gpu* g) {
+    if (g->tc_ready) return cudaSuccess;
+    cudaError_t e;
+    g->tc_seed = tc::seed_for(g->seed_idx);
+    const std::vector<uint64_t> table = tc::hash_table(g->tc_seed);
+    for (int kind = 0; kind < 2; ++kind) {
+        const std::vector<uint8_t> pool = tc::pack_pool(g->tc_seed, kind, table.data());
+        if ((e = cudaMalloc(&g->tc_pool[kind], pool.size())) != cudaSuccess) return e;
+        if ((e = cudaMemcpy(g->tc_pool[kind], pool.data(), pool.size(), cudaMemcpyHostToDevice)) != cudaSuccess) return e;
+    }
+    auto ctl = std::make_unique<TcCtl>();
+    memset(ctl.get(), 0, sizeof(TcCtl));
+    for (auto& kind : ctl->rec) for (auto& r : kind) r.first_bad = ~0u;
+    ctl->t_start_ns = ~0ull;
+    if ((e = cudaMalloc(&g->tc_ctl, sizeof(TcCtl))) != cudaSuccess) return e;
+    if ((e = cudaMemcpy(g->tc_ctl, ctl.get(), sizeof(TcCtl), cudaMemcpyHostToDevice)) != cudaSuccess) return e;
+    if ((e = cudaHostAlloc(&g->tc_out_h, sizeof(TcOut), cudaHostAllocMapped)) != cudaSuccess) return e;
+    memset(g->tc_out_h, 0, sizeof(TcOut));
+    if ((e = cudaHostGetDevicePointer(&g->tc_out_d, g->tc_out_h, 0)) != cudaSuccess) return e;
+    if ((e = cudaMalloc(&g->tc_c, sizeof(float) * tc::kM * tc::kN)) != cudaSuccess) return e;
+    if ((e = cudaEventCreate(&g->tc_e0)) != cudaSuccess) return e;
+    if ((e = cudaEventCreate(&g->tc_e1)) != cudaSuccess) return e;
+    if ((e = cudaFuncSetAttribute(tc_check<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTcSmem)) != cudaSuccess) return e;
+    if ((e = cudaFuncSetAttribute(tc_check<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTcSmem)) != cudaSuccess) return e;
+    g->tc_ready = true;
+    return cudaSuccess;
+}
+
+static void tc_free(Gpu* g) {
+    for (uint8_t*& p : g->tc_pool) { if (p) cudaFree(p); p = nullptr; }
+    if (g->tc_ctl) cudaFree(g->tc_ctl);
+    if (g->tc_out_h) cudaFreeHost(g->tc_out_h);
+    if (g->tc_c) cudaFree(g->tc_c);
+    if (g->tc_e0) cudaEventDestroy(g->tc_e0);
+    if (g->tc_e1) cudaEventDestroy(g->tc_e1);
+    g->tc_ctl = nullptr; g->tc_out_h = nullptr; g->tc_c = nullptr; g->tc_e0 = g->tc_e1 = nullptr;
+    g->tc_ready = false;
+}
+
+struct TcJob {
+    cudaError_t ce = cudaSuccess;
+    unsigned long long seq = 0;
+    uint32_t tiles = 0;
+    bool timed = false;
+    float ms = 0;
+};
+
+static TcParams tc_params(Gpu* g, int kind, uint32_t tiles) {
+    TcParams p{};
+    p.pool = g->tc_pool[kind];
+    p.desc_base = tc::smem_desc_base(kind == 0 ? 2 : 1);
+    p.idesc = tc::instr_desc(kind);
+    p.tiles = tiles;
+    p.check = g->tc_check_no;
+    p.fixed_comb = -1;
+    p.fault_sm = -1;
+    p.ctl = g->tc_ctl;
+    p.out = g->tc_out_d;
+    return p;
+}
+
+// Enqueue one check (bf16 then e4m3, one CTA per SM each) on g's stream; g's device is current.  The e4m3 launch
+// publishes both kinds' records and the sequence number.
+static void tc_issue(Gpu* g, TcJob* r) {
+    r->seq = ++g->tc_seq;
+    TcParams p = tc_params(g, 0, r->tiles);
+    p.seq = r->seq;
+    p.fault_sm = g->tc_fault_sm;
+    p.fault_mask = g->tc_fault_mask;
+    g->tc_fault_sm = -1;
+    g->tc_fault_mask = 0;
+    if (r->timed) cudaEventRecord(g->tc_e0, g->stream);
+    tc_check<0><<<(int)g->sms, kTcThreads, kTcSmem, g->stream>>>(p);
+    p = tc_params(g, 1, r->tiles);
+    p.seq = r->seq;
+    p.publish = 1;
+    tc_check<1><<<(int)g->sms, kTcThreads, kTcSmem, g->stream>>>(p);
+    r->ce = cudaGetLastError();
+    if (r->timed) cudaEventRecord(g->tc_e1, g->stream);
+    ++g->tc_check_no;
+}
+
+static inline bool tc_published(const Gpu* g, const TcJob* r) {
+    return *(volatile const unsigned long long*)&g->tc_out_h->seq == r->seq;
+}
+
+// Fold the published block into the ABI result.
+static void tc_result(Gpu* g, TcJob* r, b2dp_compute_result& o) {
+    o.seed = g->tc_seed;
+    o.sms = (int32_t)g->sms;
+    o.first_bad_sm = o.first_bad_kind = o.first_bad_tile = o.first_bad_row = -1;
+    cudaError_t e = r->ce;
+    if (e == cudaSuccess && r->timed) {
+        e = cudaEventSynchronize(g->tc_e1);
+        if (e == cudaSuccess) e = cudaEventElapsedTime(&r->ms, g->tc_e0, g->tc_e1);
+    }
+    if (e != cudaSuccess) { o.err = B2DP_E_CUDA; o.healthy = 0; return; }
+    std::atomic_thread_fence(std::memory_order_acquire);
+    TcOut out;
+    memcpy(&out, (const void*)g->tc_out_h, sizeof out);
+    if (out.seq != r->seq) { o.err = B2DP_E_CUDA; o.healthy = 0; return; }
+    for (int s = 0; s < kTcMaxSm; ++s) {
+        const TcSmRec& a = out.rec[0][s];
+        const TcSmRec& b = out.rec[1][s];
+        o.tiles += (uint64_t)a.tiles + b.tiles;
+        o.bad_rows += (uint64_t)a.bad_rows + b.bad_rows;
+        if (a.ctas && b.ctas) { o.covered_mask[s / 32] |= 1u << (s % 32); ++o.sms_covered; }
+        if (a.bad_rows || b.bad_rows) {
+            o.bad_sm_mask[s / 32] |= 1u << (s % 32);
+            if (o.sms_failed++ == 0) {
+                const int k = a.bad_rows ? 0 : 1;
+                const unsigned fb = out.rec[k][s].first_bad;
+                o.first_bad_sm = s; o.first_bad_kind = k; o.first_bad_tile = (int32_t)(fb >> 8); o.first_bad_row = (int32_t)(fb & 0xff);
+            }
+        }
+    }
+    o.ms_device = (float)((double)(out.t_end_ns - out.t_start_ns) * 1e-6);
+    o.ms_event = r->timed ? r->ms : 0.f;
+    const float ms = r->timed ? r->ms : o.ms_device;
+    o.tflops = ms > 0 ? (float)((double)tc::kM * tc::kN * tc::kK * 2.0 * (double)o.tiles / ((double)ms * 1e-3) * 1e-12) : 0.f;
+    o.healthy = o.bad_rows == 0 ? 1 : 0;
+}
+
+static void tc_log(const Gpu* g, const b2dp_compute_result& o) {
+    if (o.err == B2DP_E_TIMEOUT) logf(2, "%s: tensor-core check missed its deadline", g->dev.id.c_str());
+    else if (o.err != B2DP_OK) logf(2, "%s: tensor-core check failed to run or publish", g->dev.id.c_str());
+    else if (!o.healthy)
+        logf(2, "%s: tensor-core check failed on SM %d (%s, tile %d, row %d), %llu rows bad", g->dev.id.c_str(), o.first_bad_sm,
+             o.first_bad_kind == 0 ? "bf16" : "e4m3", o.first_bad_tile, o.first_bad_row, (unsigned long long)o.bad_rows);
+    if (o.err == B2DP_OK && o.sms_covered < o.sms)
+        logf(1, "%s: tensor-core check covered %d of %d SMs (the others ran no CTA; not a verdict)", g->dev.id.c_str(), o.sms_covered, o.sms);
+}
+
+// Launch the check on every GPU in `idx` (all before waiting on any), then poll the pinned result blocks until
+// `deadline`.  A device that misses it is B2DP_E_TIMEOUT; its worker collects the launches later (inflight).
+// The caller holds probe_mu; out has one entry per GPU of the backend.
+static void tc_fanout(CudaBackend* be, const std::vector<size_t>& idx, uint32_t tiles, bool timed,
+                      std::chrono::steady_clock::time_point deadline, std::vector<b2dp_compute_result>& out) {
+    int prev_dev = -1;
+    cudaGetDevice(&prev_dev);
+    std::vector<std::shared_ptr<TcJob>> jobs(be->gpus.size());
+    std::vector<size_t> pending;
+    for (size_t i : idx) {
+        Gpu* g = be->gpus[i].get();
+        b2dp_compute_result& o = out[i];
+        cudaSetDevice(g->ordinal);
+        cudaError_t e = tc_setup(g);
+        if (e != cudaSuccess) { o.err = B2DP_E_CUDA; o.healthy = 0; logf(2, "%s: tensor-core check setup: %s", g->dev.id.c_str(), cudaGetErrorName(e)); continue; }
+        jobs[i] = std::make_shared<TcJob>();
+        jobs[i]->tiles = tiles;
+        jobs[i]->timed = timed;
+        tc_issue(g, jobs[i].get());
+        pending.push_back(i);
+    }
+    unsigned spins = 0;
+    while (!pending.empty()) {
+        for (size_t k = 0; k < pending.size();) {
+            const size_t i = pending[k];
+            Gpu* g = be->gpus[i].get();
+            TcJob* r = jobs[i].get();
+            if (r->ce == cudaSuccess && !tc_published(g, r)) {
+                if ((spins & 0x3ff) != 0x3ff) { ++k; continue; }
+                const cudaError_t q = cudaStreamQuery(g->stream);  // a kernel that faulted never publishes
+                if (q == cudaErrorNotReady) { ++k; continue; }
+                if (q != cudaSuccess) r->ce = q;
+            }
+            if (r->timed || r->ce != cudaSuccess) cudaSetDevice(g->ordinal);
+            tc_result(g, r, out[i]);
+            pending[k] = pending.back();
+            pending.pop_back();
+        }
+        if (!pending.empty() && (++spins & 0x3ff) == 0 && std::chrono::steady_clock::now() > deadline) break;
+    }
+    for (size_t i : pending) {
+        Gpu* g = be->gpus[i].get();
+        out[i].err = B2DP_E_TIMEOUT;
+        out[i].healthy = 0;
+        g->inflight.store(true);
+        post(g, [g] { cudaStreamSynchronize(g->stream); g->inflight.store(false); });
+    }
+    if (prev_dev >= 0) cudaSetDevice(prev_dev);
 }
 
 // "0-31,64-95" -> cpu_set_t
@@ -567,7 +767,8 @@ int cuda_backend_open(const CudaConfig& cfg, CudaBackend** out, std::string& err
         const int seed_idx = cfg.seed_index >= 0 ? cfg.seed_index + idx : idx;  // a helper's one device stands for unit seed_index
         g->buf.assign((size_t)cfg.slots, nullptr);
         (void)n_vec;
-        cs.push_back(post(g, [g, bytes, idx, calib, seed_idx, &errs, &where] {
+        const bool compute = cfg.compute;
+        cs.push_back(post(g, [g, bytes, idx, calib, seed_idx, compute, &errs, &where] {
             cudaError_t e;
 #define TRY(x) if ((e = (x)) != cudaSuccess) { errs[idx] = e; where[idx] = #x; return; }
             TRY(cudaStreamCreateWithFlags(&g->stream, cudaStreamNonBlocking));
@@ -609,6 +810,8 @@ int cuda_backend_open(const CudaConfig& cfg, CudaBackend** out, std::string& err
             TRY(cudaFuncSetAttribute(hbm_probe_tma<kTmaCW, kTmaTileVec, kTmaStages>,
                                      cudaFuncAttributePreferredSharedMemoryCarveout, 100));
             g->seed = 0x5EED0000u | (uint32_t)(seed_idx & 0xffff);  // SURVEY 8(d) config 2
+            g->seed_idx = seed_idx;
+            if (compute) { if ((e = tc_setup(g)) != cudaSuccess) { errs[idx] = e; where[idx] = "tensor-core check setup"; return; } }
             g->cur = 0;
             hbm_fill<256><<<(int)g->sms * 8, 256, 0, g->stream>>>(g->buf[0], g->n_vec, g->seed);
             TRY(cudaGetLastError());
@@ -683,7 +886,8 @@ int cuda_backend_open(const CudaConfig& cfg, CudaBackend** out, std::string& err
              (int)g->buf.size(), (unsigned long long)(g->n_vec * 16 >> 20), g->small_ring ? " (shrunk: HBM was short)" : "", g->gbs_cal, ref,
              cfg.min_gbs > 0 ? cfg.min_gbs : cfg.min_frac * ref);
     }
-    if (cfg.prearm && cfg.launchers < 2) {
+    if (cfg.prearm && cfg.compute) logf(1, "prearm=1 is off with compute=1: a check queued behind an armed pass would wait for the next heartbeat");
+    if (cfg.prearm && cfg.launchers < 2 && !cfg.compute) {
         be->libcuda = dlopen("libcuda.so.1", RTLD_NOW | RTLD_LOCAL);
         if (be->libcuda) {
             void* f = dlsym(be->libcuda, "cuStreamWaitValue32_v2");
@@ -751,6 +955,7 @@ void cuda_backend_close(CudaBackend* be) {
             if (g->out_h) cudaFreeHost(g->out_h);
             if (g->e0) cudaEventDestroy(g->e0);
             if (g->e1) cudaEventDestroy(g->e1);
+            tc_free(g);
             if (g->stream) cudaStreamDestroy(g->stream);
         })->wait();
         { std::lock_guard<std::mutex> l(g->mu); g->quit = true; }
@@ -952,7 +1157,7 @@ int cuda_probe(CudaBackend* be, const b2dp_probe_opts* opts, std::vector<b2dp_pr
             if (L->sleeping.load()) { std::lock_guard<std::mutex> l(L->mu); L->cv.notify_one(); }
         }
         // prearm=1: a pass with the default options may be the one that is already enqueued behind its doorbell
-        const bool can_arm = be->wait32 && variant == B2DP_PROBE_VARIANT_TMA && !timed && grid == 0 && be->cfg.busy_policy == 0;
+        const bool can_arm = be->wait32 && !be->cfg.compute && variant == B2DP_PROBE_VARIANT_TMA && !timed && grid == 0 && be->cfg.busy_policy == 0;
         std::vector<char> arm_ok(n, 0);  // decided before any pass is issued (issuing fills in r->n_vec)
         for (size_t i = 0; i < n; ++i) arm_ok[i] = can_arm && res[i]->n_vec == 0 && res[i]->advance;
         auto armable = [&](size_t i) { return arm_ok[i] != 0; };
@@ -1098,6 +1303,19 @@ int cuda_probe(CudaBackend* be, const b2dp_probe_opts* opts, std::vector<b2dp_pr
             }
         }
         be->gpus[i]->last_healthy = o.healthy;
+    }
+    if (be->cfg.compute) {  // compute=1: the tensor-core check on every GPU whose pass ran, under the same deadline
+        std::vector<size_t> idx;
+        for (size_t i = 0; i < n; ++i) if (state[i] == 1 && !be->gpus[i]->inflight.load()) idx.push_back(i);
+        std::vector<b2dp_compute_result> cr(n, b2dp_compute_result{});
+        tc_fanout(be, idx, B2DP_COMPUTE_DEFAULT_TILES, false, deadline, cr);
+        for (size_t i : idx) {
+            if (cr[i].err == B2DP_OK && cr[i].healthy) continue;
+            tc_log(be->gpus[i].get(), cr[i]);
+            out[i].flags |= B2DP_RES_COMPUTE;
+            out[i].healthy = 0;
+            be->gpus[i]->last_healthy = 0;
+        }
     }
     if (be->cfg.check_xid) {  // opt-in: a critical Xid since open fails the device whatever the pass said
         for (size_t i = 0; i < n; ++i)
@@ -1298,6 +1516,72 @@ int cuda_describe(CudaBackend* be, int device, b2dp_probe_info* o, std::string& 
     o->gbs_cal = g->gbs_cal; o->gbs_ref = g->gbs_ref.load(); o->usable = g->broken ? 0 : 1; o->via_helper = 0;
     copy_str(o->uuid, sizeof o->uuid, g->uuid);
     copy_str(o->name, sizeof o->name, g->name);
+    return B2DP_OK;
+}
+
+int cuda_compute_check(CudaBackend* be, const b2dp_compute_opts* opts, std::vector<b2dp_compute_result>& out, std::string& err) {
+    std::lock_guard<std::mutex> pl(be->probe_mu);
+    if (be->units) { err = "the tensor-core check with per-SM detail runs in-process only (probe=inproc on whole GPUs)"; return B2DP_E_UNSUPPORTED; }
+    const uint32_t tiles = opts && opts->tiles ? opts->tiles : B2DP_COMPUTE_DEFAULT_TILES;
+    if (tiles > B2DP_COMPUTE_MAX_TILES) { err = "tiles must be at most 65536"; return B2DP_E_INVAL; }
+    const uint32_t timeout_ms = opts && opts->timeout_ms ? opts->timeout_ms : 5000;
+    const bool timed = opts && (opts->flags & B2DP_COMPUTE_EVENT_TIMING);
+    const size_t n = be->gpus.size();
+    out.assign(n, b2dp_compute_result{});
+    std::vector<size_t> idx;
+    for (size_t i = 0; i < n; ++i) {
+        Gpu* g = be->gpus[i].get();
+        out[i].device = (int)i;
+        out[i].sms = (int32_t)g->sms;
+        out[i].first_bad_sm = out[i].first_bad_kind = out[i].first_bad_tile = out[i].first_bad_row = -1;
+        if (g->broken) { out[i].err = B2DP_E_CUDA; err = g->broken_reason + " on " + g->dev.id; continue; }
+        if (g->inflight.load()) { out[i].err = B2DP_E_TIMEOUT; continue; }  // an earlier pass or check is still running
+        if (g->armed) run_sync(g, [g] { probe_flush(g); });  // a check queued behind an armed stream wait would stall
+        idx.push_back(i);
+    }
+    tc_fanout(be, idx, tiles, timed, std::chrono::steady_clock::now() + std::chrono::milliseconds(timeout_ms), out);
+    for (size_t i : idx) {
+        out[i].device = (int)i;
+        if (out[i].err != B2DP_OK || !out[i].healthy || out[i].sms_covered < out[i].sms) tc_log(be->gpus[i].get(), out[i]);
+    }
+    return B2DP_OK;
+}
+
+int cuda_compute_tile(CudaBackend* be, int device, int kind, int a_set, int b_set, float* c, std::string& err) {
+    std::lock_guard<std::mutex> pl(be->probe_mu);
+    if (be->units) { err = "in-process only (probe=inproc on whole GPUs)"; return B2DP_E_UNSUPPORTED; }
+    Gpu* g = gpu_at(be, device, err);
+    if (!g) return B2DP_E_INVAL;
+    if (g->inflight.load()) { err = "an earlier pass is still running on this device"; return B2DP_E_TIMEOUT; }
+    cudaError_t ce = cudaSuccess;
+    bool published = false;
+    run_sync(g, [&] {
+        probe_flush(g);
+        if ((ce = tc_setup(g)) != cudaSuccess) return;
+        TcParams p = tc_params(g, kind, 1);
+        p.fixed_comb = a_set * tc::kSets + b_set;
+        p.c_out = g->tc_c;
+        p.seq = ++g->tc_seq;
+        p.publish = 1;
+        if (kind == 0) tc_check<0><<<1, kTcThreads, kTcSmem, g->stream>>>(p);
+        else tc_check<1><<<1, kTcThreads, kTcSmem, g->stream>>>(p);
+        if ((ce = cudaGetLastError()) != cudaSuccess) return;
+        if ((ce = cudaMemcpyAsync(c, g->tc_c, sizeof(float) * tc::kM * tc::kN, cudaMemcpyDeviceToHost, g->stream)) != cudaSuccess) return;
+        ce = cudaStreamSynchronize(g->stream);
+        published = g->tc_out_h->seq == p.seq;
+    });
+    if (ce != cudaSuccess) { err = cuda_err("tc_check", ce); return B2DP_E_CUDA; }
+    if (!published) { err = "the tile did not publish its sequence number"; return B2DP_E_CUDA; }
+    return B2DP_OK;
+}
+
+int cuda_compute_inject_fault(CudaBackend* be, int device, int sm, uint32_t mask, std::string& err) {
+    std::lock_guard<std::mutex> pl(be->probe_mu);
+    if (be->units) { err = "in-process only (probe=inproc on whole GPUs)"; return B2DP_E_UNSUPPORTED; }
+    Gpu* g = gpu_at(be, device, err);
+    if (!g) return B2DP_E_INVAL;
+    g->tc_fault_sm = sm;
+    g->tc_fault_mask = mask;
     return B2DP_OK;
 }
 

@@ -118,6 +118,7 @@ struct CudaConfig {
     uint64_t shrink_bytes = 64ull << 20;
     bool check_ecc = false;
     bool check_xid = false;
+    bool compute = false;                // compute=1: every probe pass is followed by the tensor-core check (tc_check.cuh)
     std::vector<int> break_devices;      // test hook: indices (enumeration order) whose per-GPU setup is treated as failed
 };
 int cuda_backend_open(const CudaConfig& cfg, CudaBackend** out, std::string& err);
@@ -140,6 +141,14 @@ int cuda_describe(CudaBackend*, int device, b2dp_probe_info* out, std::string& e
 // device nodes Allocate mounts for `id` beyond the three global ones (whole GPU: /dev/nvidia<minor>; MIG instance:
 // the parent's node plus its two /dev/nvidia-caps nodes); false if the id is unknown
 bool cuda_device_paths(CudaBackend*, const std::string& id, std::vector<std::string>& out);
+// ---- ctx.cpp: what the entry points kept with the CUDA half (compute.cpp) need of a context --------------------------
+CudaBackend* ctx_cuda_backend(b2dp_ctx* c);      // nullptr unless c is a cuda: context
+int ctx_fail(int code, const std::string& msg);  // record the calling thread's last error text; returns code
+
+// tensor-core check (tc_check.cuh): B2DP_E_UNSUPPORTED in helper / probe=off mode
+int cuda_compute_check(CudaBackend*, const b2dp_compute_opts* opts, std::vector<b2dp_compute_result>& out, std::string& err);
+int cuda_compute_tile(CudaBackend*, int device, int kind, int a_set, int b_set, float* c, std::string& err);
+int cuda_compute_inject_fault(CudaBackend*, int device, int sm, uint32_t mask, std::string& err);
 // xid=1: called (from a backend thread, or from b2dp_probe_inject_fault) when a device-level Xid has been latched
 void cuda_set_health_event_callback(CudaBackend*, std::function<void()> fn);
 

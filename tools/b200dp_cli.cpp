@@ -7,7 +7,7 @@
 //       -Wl,-rpath,'$ORIGIN/../k8s-device-plugin_b200' -o tools/b200dp_cli
 //
 //   b200dp_cli <backend-uri> enumerate | health | cycle [steps [idle_ms]] | probe [steps] | resources <single|mixed>
-//                            | labels <csv> | alloc <size> | p2p
+//                            | labels <csv> | alloc <size> | p2p | compute [tiles [n]]
 #include <algorithm>
 #include <chrono>
 #include <ctime>
@@ -58,6 +58,27 @@ int main(int argc, char** argv) {
         int32_t h = 0;
         b2dp_node_health(ctx, &h);
         printf("node %s\n", h ? "Healthy" : "Unhealthy");
+    } else if (cmd == "compute") {  // tensor-core check: n event-timed checks, per GPU the median ms, TFLOP/s and SMs
+        b2dp_compute_opts o{};
+        o.tiles = argc > 3 ? (uint32_t)atoi(argv[3]) : 0;
+        o.flags = B2DP_COMPUTE_EVENT_TIMING;
+        const int steps = argc > 4 ? atoi(argv[4]) : 1;
+        std::vector<b2dp_compute_result> res(devs.size());
+        std::vector<std::vector<double>> ms(devs.size());
+        bool all_ok = true;
+        for (int s = 0; s < steps; ++s) {
+            int m = 0;
+            if ((rc = b2dp_compute_check(ctx, &o, res.data(), (int)res.size(), &m)) != B2DP_OK) return die(ctx, "b2dp_compute_check", rc);
+            for (int i = 0; i < m; ++i) { ms[i].push_back(res[i].ms_event); all_ok = all_ok && res[i].healthy; }
+        }
+        for (size_t i = 0; i < res.size(); ++i) {
+            const b2dp_compute_result& r = res[i];
+            const double t = median(ms[i]);
+            printf("%s %s ms=%.4f tflops=%.1f tiles=%llu sms=%d covered=%d failed=%d bad_rows=%llu first_bad_sm=%d\n", devs[i].id,
+                   r.healthy ? "Healthy" : "Unhealthy", t, t > 0 ? 2.0 * 128 * 128 * 128 * (double)r.tiles / (t * 1e-3) * 1e-12 : 0.0,
+                   (unsigned long long)r.tiles, r.sms, r.sms_covered, r.sms_failed, (unsigned long long)r.bad_rows, r.first_bad_sm);
+        }
+        if (!all_ok) { b2dp_close(ctx); return 1; }  // a failed check is a failing exit status
     } else if (cmd == "probe" || cmd == "cycle") {
         const int steps = argc > 3 ? atoi(argv[3]) : 200;
         const int idle_ms = argc > 4 ? atoi(argv[4]) : 0;  // sleep between cycles: the production shape is a heartbeat every few seconds
